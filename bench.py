@@ -13,6 +13,8 @@ configs[1] (20 / 10k / 80k).
 A step = ONE Levenberg-Marquardt iteration: residual+Jacobian evaluation of every observation fused with the per-point
 Schur elimination (K3a/K3b), the rank sum, the dense Cholesky solve (K4), back-substitution and evaluation of the candidate.
 Every iteration evaluates all observations, so evals/s = observations * iterations / time.
+`--dump-outputs DIR` writes what the timed pass returned after its last iteration (cameras.npy [nc,6], points.npy [np,3],
+focal.npy [1], all float64) so that two builds can be compared output for output; the inputs are seeded, identical from run to run.
 """
 import argparse
 import json
@@ -26,6 +28,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "BA residual+Jacobian evals/sec"
 UNIT = "evals/s"
@@ -164,6 +167,13 @@ def run_steps(prob, capi, k, **kw):
     return tot
 
 
+def dump_outputs(out_dir, cams, pts, focal):
+    """The BA result a caller of the timed path receives, as DIR/<name>.npy (float64; cfg3: 4.8 MB in all)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in (("cameras", cams), ("points", pts), ("focal", [focal])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(x, np.float64))
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 def run_reference(args):
     """The reference's own CPU implementation of the path.  The C++ reference cannot be built (no OpenCV/Ceres/Boost in
@@ -200,8 +210,10 @@ def run_reference(args):
     if args.warmup:
         oracle.ba_solve(*a, fixed_iteration_options(oracle, args.warmup, jacobian_mode=0, num_threads=cores))
     t0 = time.perf_counter()
-    _, _, _, s = oracle.ba_solve(*a, fixed_iteration_options(oracle, args.steps, jacobian_mode=0, num_threads=cores))
+    cams, pts, focal, s = oracle.ba_solve(*a, fixed_iteration_options(oracle, args.steps, jacobian_mode=0, num_threads=cores))
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cams, pts, focal)
     value = nobs * s["num_iterations"] / dt
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * dt / max(1, s["num_iterations"]), "higher_is_better": True, "scaling": "weak",
@@ -279,6 +291,14 @@ def run_ours(args):
     flush_ms = float(s["flush_ms_total"])
     dev_ms = dev_ms_raw - flush_ms
     launches = ctx.kernel_launches - launches0
+    if args.dump_outputs:                               # outside the bracket; before the reset below discards the result
+        cams_out, pts_out, focal_out = prob.download()
+        if world > 1:                                   # every rank holds all cameras and its contiguous range of points
+            shards = [None] * world
+            dist.all_gather_object(shards, pts_out)
+            pts_out = np.concatenate(shards)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, cams_out, pts_out, focal_out)
     # Clocks and throttle reasons: NVML / nvidia-smi queries hold the driver lock for 1-40 ms on these hosts and stall the
     # kernel launches of the process they observe (measured: the 0.83 ms step became 1.2-2.2 ms, a 2-GPU step 10 ms), so the
     # sampler does not run inside the reported pass.  It runs during an IDENTICAL second pass of the same K iterations right
@@ -554,7 +574,11 @@ def main():
     ap.add_argument("--workload", default="cfg3", choices=["cfg3", "cfg2"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stages", action="store_true", help="skip the secondary stage measurements (cfg1 replay)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the cameras, points and focal length of the last timed iteration as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -5,15 +5,17 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REQUIRED = ("impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
             "dtype", "data", "config", "cpu_baseline", "e2e")
 
 
-def _run(extra_env=None):
+def _run(extra_env=None, extra_args=()):
     env = dict(os.environ); env.update(extra_env or {})
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1", "--workload", "cfg2"],
-                       capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1", "--workload", "cfg2",
+                        *extra_args], capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
     assert r.returncode == 0, r.stderr
     return [l for l in r.stdout.splitlines() if l.strip()]
 
@@ -35,3 +37,27 @@ def test_reference_arm_prints_one_contract_line():
 
 def test_reference_arm_other_ranks_exit_quietly():
     assert _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}) == []
+
+
+def test_reference_arm_dumps_the_timed_result(tmp_path, oracle):
+    """--dump-outputs: the cameras, points and focal length after the 2 timed LM iterations, which start from the seeded problem."""
+    assert len(_run(extra_args=("--dump-outputs", str(tmp_path / "out")))) == 1
+    out = {n: np.load(tmp_path / "out" / f"{n}.npy") for n in ("cameras", "points", "focal")}
+    from sfm_toy_library_b200 import synth
+    p = synth.make_ba_problem(seed=0, **synth.BA_CONFIGS["cfg2"])
+    o = oracle.ba_default_options(max_num_iterations=2, max_solver_time_in_seconds=0.0, function_tolerance=-1.0, parameter_tolerance=-1.0,
+                                  gradient_tolerance=-1.0, jacobian_mode=0, num_threads=1)
+    cams, pts, f, s = oracle.ba_solve(p["cams"], p["pts"], p["focal"], p["obs_xy"], p["obs_cam"], p["pt_off"], o)
+    assert s["num_iterations"] == 2
+    assert all(x.dtype == np.float64 for x in out.values())
+    assert out["cameras"].shape == (20, 6) and out["points"].shape == (10_000, 3) and out["focal"].shape == (1,)
+    assert np.abs(out["cameras"] - p["cams"]).max() > 1e-6                     # the solver moved the cameras
+    np.testing.assert_allclose(out["cameras"], cams, rtol=0, atol=1e-9)
+    np.testing.assert_allclose(out["points"], pts, rtol=0, atol=1e-9 * np.abs(pts).max())
+    assert abs(out["focal"][0] - f) < 1e-9 * f
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr and r.stdout == ""
